@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's arm (one process per GPU under torchrun)
     python bench.py --impl reference --steps K --warmup W    # the UNMODIFIED reference's CPU path on the host cores
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's outputs, DIR/<name>.npy
 
 Definitions (DESIGN.md section 4):
   * workload  = config C3 of BASELINE.json: DiffusionModelUNet 3-D (256, 256, 512), attention (F, F, T), heads
@@ -22,9 +23,9 @@ Definitions (DESIGN.md section 4):
                 ControlNet + classifier-free guidance), each with its wall clock through the public API, algorithmic
                 TFLOP/s and (N = 1) the reference's CPU leg.
   * weak scaling: every GPU samples its own volume; the only collective is one all_gather of the finished samples.
-  * reference arm / cpu_baseline: the unmodified reference installed under baseline/_ref (oracle/make_ref.sh; MONAI's
+  * reference arm / cpu_baseline: the unmodified reference installed under oracle/_ref (oracle/make_ref.sh; MONAI's
                 layer wrappers come from oracle/monai_shim because MONAI is not installable offline), run through its
-                own DiffusionInferer.sample on the host cores; the oracle port only if baseline/_ref is absent.
+                own DiffusionInferer.sample on the host cores; the oracle port only if oracle/_ref is absent.
 """
 from __future__ import annotations
 
@@ -101,12 +102,12 @@ def build_model_state(seed=0):
 # ---------------------------------------------------------------------------------------------------------------
 # reference / CPU arm
 # ---------------------------------------------------------------------------------------------------------------
-REF_DIR = ROOT / "baseline" / "_ref"
+REF_DIR = ROOT / "oracle" / "_ref"
 
 
 def import_reference():
-    """The unmodified reference from baseline/_ref (pip-installed from /root/reference by oracle/make_ref.sh) on top
-    of the MONAI shim.  Returns the `generative` package or None when it did not travel."""
+    """The unmodified reference from oracle/_ref (pip-installed by oracle/make_ref.sh) on top of the MONAI shim.
+    Returns the `generative` package or None when it is not installed."""
     if not (REF_DIR / "generative" / "__init__.py").exists():
         return None
     mine = sys.modules.get("generative")
@@ -200,8 +201,8 @@ def run_reference(args):
         return
     model = build_model_state()
     value, sec, cores, kind = cpu_c3_steps(model.state_dict(), args.steps, args.warmup)
-    what = ("the unmodified reference (baseline/_ref) through its DiffusionInferer.sample" if kind == "reference"
-            else "oracle port of the reference CPU path (baseline/_ref absent)")
+    what = ("the unmodified reference (oracle/_ref) through its DiffusionInferer.sample" if kind == "reference"
+            else "oracle port of the reference CPU path (oracle/_ref absent)")
     sample = (f"{what}: UNet forward + DDIM step on 1x1x{'x'.join(map(str, CPU_VOLUME))} "
               f"(the full 160x224x160 volume needs ~60 GB of fp32 activations and 2x29.9 GiB attention scores on CPU), "
               f"{args.steps} steps after {args.warmup} warm-up, {cores} threads")
@@ -218,7 +219,7 @@ def run_reference(args):
 
 
 def cpu_other_configs(states):
-    """Bounded CPU legs of C2 / C4 / C5 through the reference (baseline/_ref), a few seconds each; None without it."""
+    """Bounded CPU legs of C2 / C4 / C5 through the reference (oracle/_ref), a few seconds each; None without it."""
     import torch
     if import_reference() is None:
         return {}
@@ -376,6 +377,25 @@ class Instrument:
 
     def ms(self, key):
         return sum(a.elapsed_time(b) for a, b in self.ev[key])
+
+
+DUMP_BYTES = 60 << 20          # of array data: with the .npy headers, under 64 MB (10^6 bytes) in all
+
+
+def dump_outputs(outdir, arrays):
+    """Write each tensor as <outdir>/<name>.npy in float32.  Past DUMP_BYTES in all, each one is cut to a fixed, seeded
+    sample of its flattened elements (the same positions on every run), an equal share of DUMP_BYTES each."""
+    import numpy as np
+    import torch
+    os.makedirs(outdir, exist_ok=True)
+    total = sum(a.numel() * 4 for a in arrays.values())
+    share = DUMP_BYTES // (4 * len(arrays))
+    for name, a in arrays.items():
+        a = a.detach().float().cpu()
+        if total > DUMP_BYTES and a.numel() > share:
+            idx = torch.randperm(a.numel(), generator=torch.Generator().manual_seed(0))[:share].sort().values
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(outdir, f"{name}.npy"), a.numpy())
 
 
 def time_calls(fn, n, sync):
@@ -565,6 +585,7 @@ def run_b200(args):
     barrier()
     inst.stop()
     ms_local = e0.elapsed_time(e1)
+    dumped = {"sample": x.cpu()} if args.dump_outputs and rank == 0 else None     # what this rank's last step returned
     clock_line = clocks.stop() if rank == 0 else None
     ms_total, per_rank = ms_local, [ms_local / args.steps]
     if world > 1:
@@ -615,7 +636,7 @@ def run_b200(args):
         if world == 1 and not args.no_cpu_baseline:
             v, sec, cores, kind = cpu_c3_steps(c3_state, 5, 1)
             cpu_line = {"value": v, "unit": "voxels/s", "cores": cores, "kind": kind,
-                        "sample": f"{'the unmodified reference (baseline/_ref)' if kind == 'reference' else 'oracle port'}: "
+                        "sample": f"{'the unmodified reference (oracle/_ref)' if kind == 'reference' else 'oracle port'}: "
                                   f"UNet forward + DDIM step on 1x1x{'x'.join(map(str, CPU_VOLUME))}, 5 steps after 1 "
                                   f"warm-up ({sec:.2f} s/step), {cores} threads"}
             if others is not None:
@@ -669,6 +690,8 @@ def run_b200(args):
             "other_configs": others,
         }
         print(json.dumps(line))
+    if dumped is not None:
+        dump_outputs(args.dump_outputs, dumped)
     if world > 1:
         dist.destroy_process_group()
 
@@ -683,7 +706,11 @@ def main():
     ap.add_argument("--volume", type=int, nargs=3, default=None, help="override the C3 volume (debug only)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-other-configs", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed as DIR/<name>.npy (float32, at most 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 0)
     if args.impl == "reference":
         run_reference(args)

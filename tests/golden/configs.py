@@ -150,7 +150,8 @@ C1_STEPS = 4
 def recipe_state_dict(module, seed=2024):
     """Deterministic, implementation-independent weights: every floating tensor of ``module.state_dict()`` (keys in
     sorted order) is drawn from one seeded CPU generator — matrices / filters ~ N(0, 1/fan_in), norm scales ~ 1 +
-    0.1 N(0,1), biases ~ 0.1 N(0,1).  Loads the result into ``module`` and returns it."""
+    0.1 N(0,1), biases ~ 0.1 N(0,1); integer buffers and attention masks keep their values.  Loads the result into
+    ``module`` and returns it."""
     import math
 
     import torch
@@ -159,7 +160,7 @@ def recipe_state_dict(module, seed=2024):
     out = {}
     for k in sorted(sd):
         t = sd[k]
-        if not t.is_floating_point():
+        if not t.is_floating_point() or k.endswith("causal_mask"):
             out[k] = t.clone()
         elif t.dim() > 1:
             out[k] = torch.randn(t.shape, generator=g) / math.sqrt(t[0].numel())

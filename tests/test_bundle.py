@@ -172,10 +172,10 @@ def test_bundle_config_runs_reference_syntax_cpu(monkeypatch, tmp_path):
 
 
 def test_reference_inference_json_parses_when_present():
-    """The unmodified bundle config (only in the build container) resolves its network definitions on this package."""
-    path = Path("/root/reference/model-zoo/models/brain_image_synthesis_latent_diffusion_model/configs/inference.json")
-    if not path.exists():
-        pytest.skip("reference tree not present")
+    """The unmodified bundle config (configs/inference.json of the model zoo's
+    brain_image_synthesis_latent_diffusion_model, stored as tests/golden/brain_ldm_inference.json) resolves its network
+    definitions on this package."""
+    path = GOLD / "brain_ldm_inference.json"
     from generativemodels_b200.bundle import BundleConfig, Sampler
     from generativemodels_b200.networks.nets import AutoencoderKL, DiffusionModelUNet
     from generativemodels_b200.networks.schedulers import DDIMScheduler
